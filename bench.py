@@ -2,12 +2,17 @@
 """Headline benchmark: UNITER-base encoder fwd+bwd samples/s (BASELINE.json configs[1] = C2).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dtype bf16|fp16]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one synthetic batch per GPU: H2D (e2e leg only),
 UniterModel forward (embeddings + 12 BertLayers on packed tokens) + MLM head + loss, backward,
 and for N > 1 the gradient allreduce (NCCL, mean) — weak scaling, 64 samples per GPU.
 Prints ONE JSON line on rank 0 (contract in the task statement; extra keys: roofline,
 cpu_baseline, clocks, e2e, gpu_launches, breakdown).
+
+`--dump-outputs DIR` writes what the last timed step computed (see dump_outputs) so that two
+builds can be compared output for output: the inputs, weights and dropout seeds are fixed, so the
+same arguments give the same inputs on every run.
 
 `--impl reference` times the CPU restatement of the reference path (oracle/, kind "port" — the
 reference is Python and cannot travel to the GPU box) on the host cores, bounded sample.
@@ -85,7 +90,47 @@ def parse():
                          "micro-batches of <= 5120 padded tokens; c5: UNITER-base ITM "
                          "hard-negative iteration (400-pair no-grad scoring + 32-pair train step, both directions)")
     ap.add_argument("--layers", type=int, default=0, help=argparse.SUPPRESS)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the loss and the gradients of the last timed step as "
+                         "DIR/<name>.npy (float32 / float64, a fixed sample of each large gradient); the GPU "
+                         "arm only (--impl ours)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU arm computed (--impl ours)")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.config == "c5" and int(os.environ.get("WORLD_SIZE", "1")) > 1 and args.steps % 8:
+        ap.error("c5 on N > 1 GPUs: --steps must be a multiple of 8 (one all-reduce per 8 iterations)")
+    return args
+
+
+DUMP_SAMPLE = 1 << 16      # entries kept of each larger gradient: ~21 MB in all for c2 / c3 / c5, ~40 MB for c4
+
+
+def dump_outputs(out_dir, loss, model):
+    """What a caller of the timed step receives from its last step: the loss (loss.npy; c5: the
+    text->images and image->texts losses) and every parameter gradient, zeros for a parameter the
+    step left without one.  A gradient of at most DUMP_SAMPLE entries is written whole as
+    grad.<parameter>.npy; of a larger one, the entries of the flattened gradient at DUMP_SAMPLE indices
+    torch.randint draws from a CPU generator seeded with the first 8 hex digits of the parameter
+    name's SHA-1.  grad_norms.npy holds the float64 L2 norm of each full gradient, in
+    named_parameters() order."""
+    import hashlib
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    if isinstance(loss, (list, tuple)):
+        loss = torch.stack([l.reshape(()) for l in loss])
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().cpu().numpy())
+    norms = []
+    for name, p in model.named_parameters():
+        g = (p.grad if p.grad is not None else torch.zeros_like(p)).detach().reshape(-1)
+        norms.append(g.double().norm().item())
+        if g.numel() > DUMP_SAMPLE:
+            seed = int(hashlib.sha1(name.encode()).hexdigest()[:8], 16)
+            idx = torch.randint(0, g.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(seed))
+            g = g[idx.to(g.device)]
+        np.save(os.path.join(out_dir, "grad.%s.npy" % name), g.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "grad_norms.npy"), np.array(norms, dtype=np.float64))
 
 
 def algorithmic_flops(lens, NL, H):
@@ -379,7 +424,14 @@ def bench_c3(args, real_out, rank, world, local_rank):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_res = timed(one_step, args.steps) / args.steps
+    last_loss = [None]
+
+    def timed_step(i):
+        last_loss[0] = one_step(i)
+
+    ms_res = timed(timed_step, args.steps) / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_loss[0], model)
     loss_host = torch.zeros(1, dtype=torch.float32).pin_memory()
 
     def e2e(i):
@@ -550,7 +602,7 @@ def bench_c5(args, real_out, rank, world, local_rank):
             ms = t.item()
         return ms
 
-    steps = max(TBS, (args.steps // TBS) * TBS)
+    steps = args.steps
     resident = [to_device(hb) for hb in host[0]]
     for i in range(max(args.warmup, 3)):
         iteration(i, resident)
@@ -558,8 +610,15 @@ def bench_c5(args, real_out, rank, world, local_rank):
     if rank == 0:
         sampler.start()
     launches0 = lib.ub200_launch_count()
-    ms_res = timed(lambda i: iteration(i, resident), steps) / steps
+    last_loss = [None]
+
+    def timed_it(i):
+        last_loss[0] = iteration(i, resident)
+
+    ms_res = timed(timed_it, steps) / steps
     launches = (lib.ub200_launch_count() - launches0) // steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_loss[0], model)
     prefetch(0)
     for i in range(n_host):
         iteration(i)
@@ -627,7 +686,7 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        nst = max(1, min(args.steps, 3))
+        nst = args.steps
         r = cpu_reference_run(args, nst, 1, args.cpu_sample)
         cb = {"value": r["value"], "unit": "samples/s", "cores": r["cores"], "host_cores": r["host_cores"],
               "kind": r["kind"], "sample": r["sample"]}
@@ -767,9 +826,10 @@ def main():
                               reducer_mode="split" if ar_mode == "split" else "in-graph")
 
     def replay(bk):
-        graphed.replay(bk)
+        loss = graphed.replay(bk)
         if ar_mode == "after":
             reducer.reduce()
+        return loss
 
     def to_device(hb, stream):
         with torch.cuda.stream(stream):
@@ -829,13 +889,16 @@ def main():
         if rank == 0:
             sampler.start()
         cpu_t = [0.0]
+        last_loss = [None]
 
         def timed_step(i):
             t0 = time.perf_counter()
-            step_resident(i)
+            last_loss[0] = step_resident(i)
             cpu_t[0] += time.perf_counter() - t0
 
         ms_total = timed(timed_step, args.steps)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, last_loss[0], model)
         cpu_enqueue_ms = cpu_t[0] / args.steps * 1e3   # host time to enqueue one step (no sync inside)
         if graphed is not None:
             launches = sum(b.launches for b in bks) // nt     # libub200 kernels inside one replay of a graph

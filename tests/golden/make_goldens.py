@@ -16,6 +16,11 @@ Cases (SURVEY.md §8c):
            of data/itm.py:356-361) — embedding output, bit-exact row selection
   heads    VQA logits / MLM scores / ITM scores through the reference heads on top of the
            reference encoder
+  reference_heads  MRFR / MRC outputs, the rows and loss of a hard-negative ITM step, and the
+           logits, losses and gradients (see grad_rows) of a multi-task pre-training step, all through
+           the reference heads (tests/test_reference_heads_gpu.py)
+  reference_schema.json  state-dict keys and shapes of the reference heads, and the model configs
+           the reference ships (tests/test_boundary_cpu.py)
 """
 import os
 import sys
@@ -425,6 +430,157 @@ def run_hardneg(rm, out_path):
     print("wrote", out_path, "%.1f KB" % (os.path.getsize(out_path) / 1024))
 
 
+def pretrain_mrm_extra(batch):
+    """Masked-region inputs of the MRFR / MRC tasks (model/pretrain.py:135-154, :201-229) for one
+    synth_batch, seeded: img_masks, img_mask_tgt, feat_targets (fp16-rounded), label_targets."""
+    gen = torch.Generator().manual_seed(8)
+    img_masks = torch.rand(batch["img_feat"].shape[:2], generator=gen) < 0.4
+    for i, nb in enumerate(batch["num_bbs"]):
+        img_masks[i, nb:] = False
+    img_masks[0, 0] = True
+    img_mask_tgt = torch.zeros_like(batch["attn_masks"], dtype=torch.bool)
+    for i, tl in enumerate(batch["txt_lens"]):
+        nb = batch["num_bbs"][i]
+        img_mask_tgt[i, tl:tl + nb] = img_masks[i, :nb]
+    n = int(img_masks.sum())
+    return {"img_masks": img_masks, "img_mask_tgt": img_mask_tgt,
+            "feat_targets": batch["img_feat"][img_masks].half().float(),
+            "label_targets": torch.softmax(torch.randn(n, 11, generator=gen), -1)}
+
+
+def library_pretrain_inputs(use_index):
+    """(base batch, the same batch with masked regions, keys the heads read) of the multi-task
+    pre-training comparison; without `use_index` the fixed-shape row lists are left out."""
+    from uniter_b200.synth import synth_batch, synth_mrm
+    base = synth_batch(5, 5, 9, 4, 8, seed=17, img_dim=64, vocab_size=2000, mlm_prob=0.3)
+    mb = synth_mrm(base, mask_prob=0.3, label_dim=11, seed=3)
+    keys = [k for k, v in mb.items() if torch.is_tensor(v)]
+    if not use_index:
+        keys = [k for k in keys if k not in ("mlm_index", "mlm_targets", "mrm_index", "mrm_valid", "mrm_inv_n")]
+    return base, mb, keys
+
+
+LIBRARY_PRETRAIN_TASKS = ("mlm", "mrfr", "mrc", "mrc-kl", "itm")
+LIBRARY_PRETRAIN_GRADS = (
+    "feat_regress.net.0.weight", "feat_regress.net.2.weight", "feat_regress.bias",
+    "region_classifier.net.0.weight", "region_classifier.net.3.weight", "region_classifier.net.3.bias",
+    "itm_output.weight", "itm_output.bias", "uniter.pooler.dense.weight", "uniter.pooler.dense.bias",
+    "cls.predictions.transform.dense.weight", "cls.predictions.bias",
+    "uniter.embeddings.word_embeddings.weight", "uniter.img_embeddings.img_linear.weight",
+    "uniter.img_embeddings.mask_embedding.weight", "uniter.encoder.layer.1.output.dense.weight")
+
+
+def grad_rows(g, key, whole=65536, budget=16384):
+    """Rows of gradient `g` to store: every row when it holds <= `whole` entries (all but the
+    word-embedding table), else `budget` entries: the largest-norm half (the rows the embedding
+    lookup touches) plus a seeded sample of the rest (the tied decoder's dense part)."""
+    import hashlib
+    if g.dim() < 2 or g.numel() <= whole:
+        return torch.arange(g.size(0))
+    n = max(2, budget // g[0].numel())
+    top = g.norm(dim=1).topk(n // 2)[1]
+    rest = torch.ones(g.size(0), dtype=torch.bool)
+    rest[top] = False
+    gen = torch.Generator().manual_seed(int(hashlib.sha1(key.encode()).hexdigest()[:8], 16) & 0x7FFFFFFF)
+    pick = rest.nonzero().squeeze(1)[torch.randperm(int(rest.sum()), generator=gen)[:n - n // 2]]
+    return torch.cat([top, pick]).sort()[0]
+
+
+def run_reference_heads(rm, out_path):
+    """The reference's own task heads over the reference encoder (CPU fp32, weights rounded to fp16):
+    what tests/test_reference_heads_gpu.py compares the drop-in heads on the GPU with."""
+    import model.itm as ritm
+    import model.pretrain as rpre
+    from uniter_b200.synth import seeded_state, synth_batch
+
+    def set_dropout_zero(m):
+        for _, mod in m.named_modules():
+            if isinstance(mod, torch.nn.Dropout):
+                mod.p = 0.0
+
+    cfg = rm.UniterConfig(**TINY)
+    rec = {}
+    # --- pre-training heads, MRFR / MRC on the heads batch
+    pre = rpre.UniterForPretraining(cfg, 64, 11)
+    st = seeded_state({k: tuple(v.shape) for k, v in pre.state_dict().items()}, seed=4)
+    pre.load_state_dict({k: v.half().float() for k, v in st.items()}, strict=True)
+    pre.eval()
+    batch = synth_batch(3, 5, 9, 4, 8, seed=7, img_dim=64, vocab_size=2000, mlm_prob=0.3)
+    cb = {k: v for k, v in batch.items() if torch.is_tensor(v)}
+    cb["img_feat"] = cb["img_feat"].half().float()
+    cb["img_pos_feat"] = cb["img_pos_feat"].half().float()
+    extra = pretrain_mrm_extra(batch)
+    with torch.no_grad():
+        for task in ("mrfr", "mrc"):
+            rec["pre/" + task] = pre(dict(cb, **extra), task=task, compute_loss=False).numpy()
+    # --- hard-negative ITM: rows mined and loss of one train step, both directions
+    mod = ritm.UniterForImageTextRetrievalHardNeg(cfg, 16, hard_size=3)
+    st = seeded_state({k: tuple(v.shape) for k, v in mod.state_dict().items()}, seed=6)
+    mod.load_state_dict({k: v.half().float() for k, v in st.items()}, strict=True)
+    mod.train()
+    set_dropout_zero(mod)
+    for sf in ("t", "i"):
+        cbatch, _ = hardneg_inputs(sf, seed=77)
+        cbatch["img_feat"] = cbatch["img_feat"].half().float()
+        cbatch["img_pos_feat"] = cbatch["img_pos_feat"].half().float()
+        picked = {}
+        orig = mod._get_hard_batch
+        mod._get_hard_batch = lambda bt, sc, sfrom, _o=orig: picked.setdefault("rows", _o(bt, sc, sfrom))
+        loss = mod(cbatch, sample_from=sf, compute_loss=True)
+        mod._get_hard_batch = orig
+        key = "img_feat" if sf == "t" else "input_ids"
+        rec["hardneg/%s/%s" % (sf, key)] = picked["rows"][key].float().numpy()
+        rec["hardneg/%s/loss" % sf] = loss.detach().numpy()
+    # --- multi-task pre-training step: logits, per-element losses, gradients of the summed loss
+    ref = rpre.UniterForPretraining(cfg, 64, 11)
+    st = seeded_state({k: tuple(v.shape) for k, v in ref.state_dict().items()}, seed=4)
+    ref.load_state_dict({k: v.half().float() for k, v in st.items()}, strict=True)
+    ref.eval()
+    base, mb, keys = library_pretrain_inputs(use_index=False)
+    cb = {k: (mb[k].half().float() if mb[k].is_floating_point() else mb[k]) for k in keys}
+    cb["targets"] = torch.tensor([1, 0, 1, 1, 0])
+    cb["ot_inputs"] = None
+    plain = dict(cb, img_feat=base["img_feat"].half().float())
+    total = 0.0
+    for task in LIBRARY_PRETRAIN_TASKS:
+        bc = plain if task in ("mlm", "itm") else cb
+        with torch.no_grad():
+            want = ref(bc, task=task, compute_loss=False)
+        lw = ref(bc, task=task, compute_loss=True)
+        want = want[0] if isinstance(want, tuple) else want
+        lw = lw[0] if isinstance(lw, tuple) else lw
+        rec["library/%s/logits" % task] = want.numpy()
+        rec["library/%s/loss" % task] = lw.detach().numpy()
+        total = total + lw.float().mean()
+    total.backward()
+    params = dict(ref.named_parameters())
+    for name in LIBRARY_PRETRAIN_GRADS:
+        g = params[name].grad
+        rows = grad_rows(g, name)
+        rec["library/grad_rows/" + name] = rows.numpy()
+        rec["library/grad/" + name] = g[rows].numpy()
+    np.savez_compressed(out_path, **rec)
+    print("wrote", out_path, "%.1f KB" % (os.path.getsize(out_path) / 1024))
+
+
+def run_reference_schema(rm, rvqa, rpre, out_path):
+    """State-dict schema of the reference's own heads over the reference encoder and the model
+    configs it ships (config/uniter-{base,large}.json)."""
+    import json
+    cfg = rm.UniterConfig(**TINY)
+    rec = {"configs": {}}
+    for name in ("uniter-base.json", "uniter-large.json"):
+        with open(os.path.join(REF, "config", name)) as fh:
+            rec["configs"][name] = json.load(fh)
+    for tag, mod in (("vqa", rvqa.UniterForVisualQuestionAnswering(cfg, 64, 17)),
+                     ("pretraining", rpre.UniterForPretraining(cfg, 64, 11))):
+        rec[tag] = {k: list(v.shape) for k, v in mod.state_dict().items()}
+    with open(out_path, "w") as fh:
+        json.dump(rec, fh, indent=1, sort_keys=True)
+        fh.write("\n")
+    print("wrote", out_path, "%.1f KB" % (os.path.getsize(out_path) / 1024))
+
+
 def run_adamw(out_path):
     """4 steps of the reference's own AdamW (optim/adamw.py) + clip_grad_norm_ on seeded fp32
     tensors: two param groups (decay 0.01 / 0), a linear-warmup lr per step, gradient clipping at
@@ -499,6 +655,8 @@ def main():
     run_case(rm, LARGE_L1, 2048, lg, os.path.join(HERE, "large_l1.npz"), full_grads=False)
     run_heads(rm, rvqa, rpre, os.path.join(HERE, "heads_tiny.npz"))
     run_hardneg(rm, os.path.join(HERE, "hardneg.npz"))
+    run_reference_heads(rm, os.path.join(HERE, "reference_heads.npz"))
+    run_reference_schema(rm, rvqa, rpre, os.path.join(HERE, "reference_schema.json"))
     run_adamw(os.path.join(HERE, "adamw.npz"))
     run_batching(os.path.join(HERE, "batching.npz"))
     run_itm_batching(os.path.join(HERE, "itm_batching.npz"))

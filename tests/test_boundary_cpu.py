@@ -4,8 +4,9 @@
   * ctypes struct mirrors have the size the C compiler gives the header's structs;
   * UniterConfig / UniterModel keep the reference's constructor, parameter schema, from_pretrained
     renames and error conventions (SURVEY.md §8b-B1);
-  * the reference's own task heads accept our UniterModel when /root/reference is present
-    (construction + state-dict level; compute needs the GPU);
+  * the reference's own task heads accept our UniterModel where the reference sources are staged,
+    and the library's heads keep their state-dict schema and weight tying
+    (tests/golden/reference_schema.json; construction + state-dict level, compute needs the GPU);
   * the product never silently falls back: forward on CPU / fp32 raises.
 """
 import ctypes as C
@@ -13,15 +14,16 @@ import json
 import os
 import re
 import subprocess
-import sys
 import tempfile
 
 import pytest
 import torch
 
+from oracle import ref_loader
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HEADER = os.path.join(ROOT, "include", "ub200.h")
-REF = "/root/reference"
+SCHEMA = os.path.join(ROOT, "tests", "golden", "reference_schema.json")
 
 
 @pytest.fixture(scope="module")
@@ -111,11 +113,14 @@ def test_config_matches_reference_semantics(tmp_path):
     c = UniterConfig.from_json_file(str(p))
     assert c.hidden_size == 768 and c.extra_key == 7        # every JSON key is copied (model/model.py:89-102)
     assert json.loads(c.to_json_string())["vocab_size"] == 28996
-    for name in ("uniter-base.json", "uniter-large.json"):
-        path = os.path.join(REF, "config", name)
-        if os.path.exists(path):
-            c = UniterConfig.from_json_file(path)
-            assert c.hidden_size == 64 * c.num_attention_heads
+    with open(SCHEMA) as fh:
+        configs = json.load(fh)["configs"]          # the reference's config/uniter-{base,large}.json
+    assert sorted(configs) == ["uniter-base.json", "uniter-large.json"]
+    for name, body in configs.items():
+        path = tmp_path / name
+        path.write_text(json.dumps(body))
+        c = UniterConfig.from_json_file(str(path))
+        assert c.hidden_size == 64 * c.num_attention_heads
 
 
 def test_state_dict_schema_and_weight_decay_names():
@@ -192,14 +197,16 @@ def test_qkv_packing_survives_dtype_casts():
     assert att.key.weight.data_ptr() == att.query.weight.data_ptr() + H * H * 2
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present")
+@pytest.mark.skipif(not ref_loader.available(), reason="reference sources not staged")
 def test_reference_heads_accept_the_drop_in_model():
     """Monkey-patch model.model.UniterModel (the INTEGRATION.md recipe) and build the reference's
-    own heads on top of it: constructor, init_weights, weight tying and state-dict keys."""
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    import make_goldens
-    rm, rvqa, rpre = make_goldens.import_reference()
+    own heads on top of it: constructor, init_weights, weight tying, and the state-dict keys and
+    shapes the same heads have over the reference encoder (reference_schema.json)."""
+    from tests.golden import make_goldens
     from uniter_b200.model import UniterModel
+    rm, rvqa, rpre = ref_loader.load("model.model", "model.vqa", "model.pretrain")
+    with open(SCHEMA) as fh:
+        want = json.load(fh)
     orig = rm.UniterModel
     try:
         for mod in (rvqa, rpre):
@@ -208,15 +215,35 @@ def test_reference_heads_accept_the_drop_in_model():
         vqa = rvqa.UniterForVisualQuestionAnswering(cfg, 64, 17)
         assert isinstance(vqa.uniter, UniterModel)
         pre = rpre.UniterForPretraining(cfg, 64, 11)
+        assert isinstance(pre.uniter, UniterModel)
         assert pre.cls.predictions.decoder.weight is pre.uniter.embeddings.word_embeddings.weight
         assert pre.feat_regress.weight is pre.uniter.img_embeddings.img_linear.weight
-        ref_keys = set(rpre.UniterForPretraining.__mro__[0](cfg, 64, 11).state_dict().keys())
-        rpre.UniterModel = orig
-        want = set(rpre.UniterForPretraining(cfg, 64, 11).state_dict().keys())
-        assert ref_keys == want
+        for tag, mod in (("vqa", vqa), ("pretraining", pre)):
+            assert {k: list(v.shape) for k, v in mod.state_dict().items()} == want[tag], tag
     finally:
         rvqa.UniterModel = orig
         rpre.UniterModel = orig
+
+
+def test_library_heads_keep_the_reference_schema():
+    """The library's own heads (uniter_b200.heads) over our UniterModel: constructor, init_weights,
+    weight tying, and the state-dict keys and shapes of the reference's heads over the reference
+    encoder (reference_schema.json)."""
+    from uniter_b200.heads import UniterForPretraining, UniterForVisualQuestionAnswering
+    from uniter_b200.model import UniterModel
+    with open(SCHEMA) as fh:
+        want = json.load(fh)
+    cfg = _tiny_cfg()
+    vqa = UniterForVisualQuestionAnswering(cfg, 64, 17)
+    assert isinstance(vqa.uniter, UniterModel)
+    pre = UniterForPretraining(cfg, 64, 11)
+    assert pre.cls.predictions.decoder.weight is pre.uniter.embeddings.word_embeddings.weight
+    assert pre.feat_regress.weight is pre.uniter.img_embeddings.img_linear.weight
+    for tag, mod in (("vqa", vqa), ("pretraining", pre)):
+        got = {k: list(v.shape) for k, v in mod.state_dict().items()}
+        assert got == want[tag], tag
+    enc = {k[len("uniter."):]: v for k, v in want["pretraining"].items() if k.startswith("uniter.")}
+    assert {k: list(v.shape) for k, v in UniterModel(cfg, 64).state_dict().items()} == enc
 
 
 def test_prefix_pack_bookkeeping_matches_mask_derived_indices():
